@@ -10,9 +10,9 @@ reference's own ``stages.main`` / ``limiter.limit`` / helpers run unmodified:
 * statsmodels.api.nonparametric.lowess -> oracle/lowess.py (the one piece of
   hot-path arithmetic that is a restatement; see that file's header).
 
-Only usable in the build container (/root/reference does not exist on the GPU
-box).  Used by oracle/make_golden.py and by the `not gpu` tests that pin
-oracle/port.py against the real reference when it is present.
+Needs a checkout of the reference (MATCHERING_REFERENCE_ROOT).  Used by the
+oracle/make_golden*.py scripts, which store what the tests compare against
+under tests/golden/.
 """
 import os
 import sys

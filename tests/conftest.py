@@ -22,14 +22,3 @@ def golden():
     def load(name):
         return np.load(os.path.join(GOLDEN, name))
     return load
-
-
-@pytest.fixture(scope="session")
-def reference_package():
-    """The unmodified reference, when /root/reference exists (build container only)."""
-    import ref_shims
-    if not ref_shims.reference_available():
-        pytest.skip("reference tree not present (GPU box)")
-    import warnings
-    warnings.simplefilter("ignore")
-    return ref_shims.import_reference()

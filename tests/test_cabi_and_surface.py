@@ -1,6 +1,7 @@
 """Host-side checks that need no GPU: the C ABI library loads and exports every symbol the header
 declares; the Python surface mirrors the reference's (Config/Result/log/process)."""
 import ctypes as C
+import json
 import os
 import re
 
@@ -76,13 +77,21 @@ def test_config_matches_reference_defaults_and_asserts():
         mg.LimiterConfig(hold_filter_order=0)
 
 
-def test_config_attribute_parity_with_reference(reference_package):
+def reference_surface():
+    """The reference's Config attributes and log codes (tests/golden/reference_surface.json, written by
+    oracle/make_golden_parity.py from the unmodified reference)."""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_surface.json")) as f:
+        return json.load(f)
+
+
+def test_config_attribute_parity_with_reference():
     import matchering_b200 as mg
-    from matchering import Config as RefConfig
-    ours, theirs = mg.Config(internal_sample_rate=48000, max_piece_size=7.5), RefConfig(internal_sample_rate=48000, max_piece_size=7.5)
-    for name, value in vars(theirs).items():
+    ref = reference_surface()
+    assert ref["config_kwargs"] == dict(internal_sample_rate=48000, max_piece_size=7.5)
+    ours = mg.Config(internal_sample_rate=48000, max_piece_size=7.5)
+    for name, value in ref["config"].items():
         if name == "limiter":
-            assert vars(ours.limiter) == vars(value)
+            assert vars(ours.limiter) == value
         else:
             assert getattr(ours, name) == value, name
 
@@ -108,10 +117,9 @@ def test_results_and_log_surface():
     assert int(Code.ERROR_VALIDATION) == 4202 and str(ModuleError(Code.ERROR_VALIDATION)).startswith("4202: Validation failed")
 
 
-def test_log_codes_match_reference(reference_package):
-    from matchering.log.codes import Code as RefCode
+def test_log_codes_match_reference():
     from matchering_b200.log import Code
-    assert {c.name: int(c) for c in Code} == {c.name: int(c) for c in RefCode}
+    assert {c.name: int(c) for c in Code} == reference_surface()["log_codes"]
 
 
 def test_wav_roundtrip_and_checker(tmp_path):

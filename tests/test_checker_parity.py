@@ -1,7 +1,10 @@
 """matchering_b200.checker against the UNMODIFIED reference's checker (matchering/checker.py:75-137):
 the clipping / limiter warning rule, the order of the checks and the rate-scaled minimum length.
-The cases' expected warnings are also written out as a golden list, so the rule stays pinned where
-the reference tree is absent (GPU box)."""
+What the reference's checker reported on these cases is stored in tests/golden/reference_surface.json
+(oracle/make_golden_parity.py)."""
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -10,6 +13,14 @@ from matchering_b200 import checker
 from matchering_b200.log import Code, ModuleError
 
 CLIP, LIM = int(Code.WARNING_TARGET_IS_CLIPPING), int(Code.WARNING_TARGET_LIMITER_IS_APPLIED)
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_surface.json")
+
+
+@pytest.fixture(scope="module")
+def reference_checker():
+    with open(GOLDEN) as f:
+        surface = json.load(f)
+    return surface["checker_warnings"], surface["checker_errors"]
 
 
 def _noise(n=6000, seed=0, scale=0.5):
@@ -23,7 +34,7 @@ def _with_peaks(peak, count, n=6000, seed=0):
     return x
 
 
-# (label, array, expected warning codes in order) -- verified against the live reference below
+# (label, array, expected warning codes in order) -- verified against the reference below
 CASES = [
     ("24-bit +FS x 20 -> clipping", _with_peaks(8388607 / 8388608, 20), [CLIP]),
     ("24-bit +FS x 8 (at the threshold, not above)", _with_peaks(8388607 / 8388608, 8), []),
@@ -45,14 +56,8 @@ def test_peak_warning_rule(label, array, expected):
 
 
 @pytest.mark.parametrize("label,array,expected", CASES, ids=[c[0] for c in CASES])
-def test_peak_warning_rule_matches_live_reference(reference_package, label, array, expected):
-    ref = reference_package
-    seen = []
-    ref.log(warning_handler=seen.append)
-    try:
-        ref.checker.check(array.copy(), 44100, ref.Config(), "target")
-    finally:
-        ref.log()
+def test_peak_warning_rule_matches_live_reference(reference_checker, label, array, expected):
+    seen = reference_checker[0][label]  # the reference's warnings on this array
     from matchering_b200.log.explanations import explain
     assert seen == [explain(Code(c), False) for c in expected]
     ours = []
@@ -64,25 +69,26 @@ def test_peak_warning_rule_matches_live_reference(reference_package, label, arra
     assert ours == seen and sr == 44100 and np.array_equal(out, array)
 
 
-def test_check_order_and_scaled_minimum_length(reference_package):
+def test_check_order_and_scaled_minimum_length(reference_checker):
     """Length is judged at the SOURCE rate against fft_size * rate // internal_rate, before channels
     and before resampling (matchering/checker.py:95-110)."""
-    ref = reference_package
-    cfg_ours, cfg_ref = mg.Config(), ref.Config()
-    from matchering.log.exceptions import ModuleError as RefError
+    ref_errors = reference_checker[1]  # what the reference's checker raised on the same two arrays
+    cfg_ours = mg.Config()
     # 3000 frames at 22050 Hz: >= 4096 * 22050 // 44100 = 2048 -> accepted by the length check, and the
     # 3-channel error comes before any resampling
     x3 = np.zeros((3000, 3))
-    for mod, cfg, err in ((checker, cfg_ours, ModuleError), (ref.checker, cfg_ref, RefError)):
-        with pytest.raises(err) as e:
-            mod.check(x3, 22050, cfg, "reference")
-        assert str(e.value).startswith(f"{int(Code.ERROR_REFERENCE_NUM_OF_CHANNELS_IS_EXCEEDED)}:")
+    with pytest.raises(ModuleError) as e:
+        checker.check(x3, 22050, cfg_ours, "reference")
+    for err in (ref_errors["three_channels_22050"], {"type": type(e.value).__name__, "message": str(e.value)}):
+        assert err["type"] == "ModuleError"
+        assert err["message"].startswith(f"{int(Code.ERROR_REFERENCE_NUM_OF_CHANNELS_IS_EXCEEDED)}:")
     # 2000 frames at 22050 Hz: below the scaled minimum
     x2 = np.zeros((2000, 2))
-    for mod, cfg, err in ((checker, cfg_ours, ModuleError), (ref.checker, cfg_ref, RefError)):
-        with pytest.raises(err) as e:
-            mod.check(x2, 22050, cfg, "target")
-        assert str(e.value).startswith(f"{int(Code.ERROR_TARGET_LENGTH_IS_TOO_SMALL)}:")
+    with pytest.raises(ModuleError) as e:
+        checker.check(x2, 22050, cfg_ours, "target")
+    for err in (ref_errors["too_short_22050"], {"type": type(e.value).__name__, "message": str(e.value)}):
+        assert err["type"] == "ModuleError"
+        assert err["message"].startswith(f"{int(Code.ERROR_TARGET_LENGTH_IS_TOO_SMALL)}:")
     # too long is judged at the source rate as well
     class Fake:  # only .shape is looked at before the error
         shape = (cfg_ours.max_length * 22050 + 1, 2)

@@ -1,9 +1,10 @@
-"""oracle/port.py pinned: against the golden vectors generated from the unmodified reference
-(always), and against the reference itself where /root/reference exists."""
+"""oracle/port.py pinned against the golden vectors generated from the unmodified reference
+(oracle/make_golden.py, oracle/make_golden_full.py, oracle/make_golden_parity.py)."""
 import numpy as np
 import pytest
 
 import port
+from make_golden_parity import EVERY, digest, identities_inputs, main_inputs, preview_inputs
 
 
 def cfg_for(npz):
@@ -52,61 +53,67 @@ def test_limiter_early_out_returns_input_object():
     assert port.limit(x, port.OracleConfig()) is x
 
 
-# ---- against the live reference (build container only) -------------------------------------------
-def test_identities_against_reference_helpers(reference_package):
-    from matchering import Config, dsp
-    from matchering.limiter import hyrax
-    from matchering.stage_helpers import match_frequencies as mf
-    rng = np.random.default_rng(5)
-    g = np.abs(rng.standard_normal(5000)) * (rng.uniform(size=5000) > 0.7)
+# ---- against the reference's outputs on the same seeded inputs (tests/golden/reference_parity.npz) ------
+def test_identities_against_reference_helpers(golden):
+    ref = golden("reference_parity.npz")
+    g, pieces, x = identities_inputs()
+    assert digest(np.concatenate([g, pieces.ravel(), x.ravel()])) == ref["identities_input_sha256"], "inputs differ from the golden's"
     for attack in (44, 45, 96):
-        want = getattr(hyrax, "__sliding_window_fast")(g, attack, "attack")
         reach = (attack + 1 if not attack & 1 else attack) - 1
-        assert np.array_equal(port.centred_max(g, reach), want)
+        assert digest(port.centred_max(g, reach)) == ref[f"attack_max_{attack}_sha256"]
     for hold in (44, 45, 96, 3):
-        want = getattr(hyrax, "__sliding_window_fast")(g, hold, "hold")
-        assert np.array_equal(port.trailing_max(g, hold), want)
-    cfg = Config()
-    att, slided = getattr(hyrax, "__process_attack")(np.copy(g), cfg)
-    k = port.limiter_coefficients(port.config_from(cfg))
-    assert np.abs(port.one_pole_forward_backward(slided, k["c"]) - att).max() < 1e-15
-    pieces = rng.standard_normal((3, 20000))
-    want = getattr(mf, "__average_fft")(pieces, 44100, 4096)
+        assert digest(port.trailing_max(g, hold)) == ref[f"hold_max_{hold}_sha256"]
+    k = port.limiter_coefficients(port.OracleConfig())
+    slided = port.centred_max(g, k["reach"])
+    assert digest(slided) == ref["attack_envelope_sha256"]
+    assert np.abs(port.one_pole_forward_backward(slided, k["c"]) - ref["attack_gain"]).max() < 1e-15
     flat = pieces.reshape(-1)
     got = port.average_spectrum(flat, 20000, np.ones(3, dtype=bool), 4096)
-    assert np.abs(got - want).max() < 1e-15
-    x = rng.standard_normal((1000, 2))
-    mid, side = dsp.lr_to_ms(x)
+    assert np.abs(got - ref["average_fft"]).max() < 1e-15
     m2, s2 = port.mid_side(x)
-    assert np.array_equal(mid, m2) and np.array_equal(side, s2)
+    assert digest(m2) == ref["mid_sha256"] and digest(s2) == ref["side_sha256"]
+
+
+def _compare_summary(y, ref, prefix, tol):
+    """y against oracle/make_golden_parity.py's summary of the reference's output: the sampled rows at
+    `tol`, and 64 block sums of y and of its square, in which every frame takes part."""
+    assert y.shape[0] == int(ref[prefix + "frames"])
+    assert np.abs(y[::EVERY] - ref[prefix + "rows"]).max() < tol
+    edges = ref[prefix + "block_edges"]
+    frames_per_block = np.diff(edges)[:, None]
+    block_sum = np.array([y[a:b].sum(axis=0) for a, b in zip(edges[:-1], edges[1:])])
+    block_sq = np.array([np.einsum("ij,ij->j", y[a:b], y[a:b]) for a, b in zip(edges[:-1], edges[1:])])
+    # a per-sample error e moves a block's mean by at most e and its mean square by at most 2*peak*e
+    peak = max(1.0, float(np.abs(y).max()))
+    assert (np.abs(block_sum - ref[prefix + "block_sum"]) / frames_per_block).max() < tol
+    assert (np.abs(block_sq - ref[prefix + "block_sumsq"]) / frames_per_block).max() < 2 * peak * tol
 
 
 @pytest.mark.parametrize("sr,seconds", [(44100, 6.0), (96000, 2.5)])
-def test_main_against_reference(reference_package, sr, seconds):
-    from matchering import Config, stages
-    n = int(sr * seconds)
-    t = port.synth_target(n, 3).astype(np.float64)
-    r = port.synth_reference(n - 777, 4).astype(np.float64)
-    cfg = Config(internal_sample_rate=sr, max_piece_size=1.0)
-    want = stages.main(t, r, cfg, True, True, True)
+def test_main_against_reference(golden, sr, seconds):
+    ref = golden("reference_parity.npz")
+    t, r = main_inputs(sr, seconds)
+    key = f"main_{sr}_"
+    assert digest(np.concatenate([t.ravel(), r.ravel()])) == ref[key + "input_sha256"], "inputs differ from the golden's"
+    cfg = port.OracleConfig(internal_sample_rate=sr, max_piece_size=1.0)
     got = port.main(t, r, cfg, True, True, True)
-    for a, b in zip(got, want):
-        assert np.abs(a - b).max() < 1e-12
+    for name, y in zip(("limited", "no_limiter", "normalized"), got):
+        _compare_summary(y, ref, key + name + "_", 1e-12)
 
 
 @pytest.mark.parametrize("n,whole", [(30000, False), (9000, True), (12000 + 4000 * 3, False)])
-def test_preview_pieces_against_reference(reference_package, monkeypatch, n, whole):
-    """oracle/port.py::preview_pieces against the unmodified create_preview (its two `save` calls captured)."""
-    from matchering import Config, Result, preview_creator
-    cfg = Config(internal_sample_rate=2000, preview_size=6, preview_analysis_step=2)
-    saved = {}
-    monkeypatch.setattr(preview_creator, "save", lambda file, arr, sr, subtype, name: saved.__setitem__(name, arr.copy()))
-    target = 2.5 * port.synth_target(n, 41).astype(np.float64)
-    result = port.synth_reference(n, 42).astype(np.float64) * (0.2 + np.abs(np.sin(np.linspace(0, 9, n))))[:, None]
-    keep_t, keep_r = target.copy(), result.copy()
-    preview_creator.create_preview(target, result, cfg, Result("t.wav", "PCM_16"), Result("r.wav", "PCM_16"))
-    index, t_piece, r_piece = port.preview_pieces(keep_t, keep_r, cfg)
-    assert np.array_equal(saved["target preview"], t_piece) and np.array_equal(saved["result preview"], r_piece)
+def test_preview_pieces_against_reference(golden, n, whole):
+    """oracle/port.py::preview_pieces against the pieces the unmodified create_preview passed to its two
+    `save` calls, bit for bit."""
+    ref = golden("reference_parity.npz")
+    target, result = preview_inputs(n)
+    key = f"preview_{n}_"
+    assert digest(np.concatenate([target.ravel(), result.ravel()])) == ref[key + "input_sha256"], "inputs differ from the golden's"
+    import matchering_b200 as mg
+    cfg = mg.Config(internal_sample_rate=2000, preview_size=6, preview_analysis_step=2)
+    index, t_piece, r_piece = port.preview_pieces(target, result, cfg)
+    for name, piece in (("target", t_piece), ("result", r_piece)):
+        assert piece.shape == tuple(ref[key + name + "_shape"]) and digest(piece) == ref[key + name + "_sha256"]
     assert (len(r_piece) == n) == whole
     if not whole:
         assert r_piece[0].tolist() == [0.0, 0.0] and r_piece[-1].tolist() == [0.0, 0.0]
